@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the coupled-cluster hot path (BASELINE.json metric: CCSD s/iter & (T) wall-s; % FP64 tensor peak; vs CPU).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--nbf 200 --nocc 20]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--nbf 200 --nocc 20] [--dump-outputs DIR]
     python bench.py --workload n2|f2|h2o|h2o-spinorb      (sample_data molecules, whole converged run; see below)
 
 One "step" = one pass of the hot path over the synthetic (nbf, nocc) system: one spin-free CCSD iteration
@@ -212,6 +212,31 @@ def mp1_triples_check(gpu, n, o, eps, src, big, chk):
             "abs_diff": diffs, "tolerance": "relative 1e-9, absolute floor 1e-15 Eh", "ok": bool(ok)}
 
 
+# ------------------------------------------------------------------------------------------------ outputs
+DUMP_T2_SAMPLE = 1 << 20   # T2 positions kept by --dump-outputs (8 MB; all of T2 is 104 MB at nbf=200/nocc=20)
+
+
+def dump_outputs(gpu, out_dir, last):
+    """--dump-outputs: what a caller of the timed path receives from its last step, as float64 .npy files, so that two
+    builds run with the same arguments (hence the same seeded inputs) can be compared output by output:
+      ccsd_iterate.npy   [E_CCSD, rms of the T2 update] (afesp_gpu_ccsd_iterate)
+      t1_diagnostic.npy  [T1 diagnostic] (afesp_gpu_ccsd_finalize)
+      ccsd_t_sums.npy    the six (T) sums (afesp_gpu_ccsd_t_spatial)
+      t1.npy             T1 (nocc, nvirt)
+      t2_sample.npy      T2 at DUMP_T2_SAMPLE distinct positions of its column-major (nocc, nocc, nvirt, nvirt) storage,
+                         drawn with a fixed seed and kept in ascending order (all of T2 when it is not larger)
+    The amplitudes are read with afesp_gpu_ccsd_finalize, which under finalize_keep_ccsd=1 copies them and changes no state."""
+    _, t1, t2 = gpu.ccsd_finalize(want_amplitudes=True)
+    t2 = t2.ravel(order="F")
+    if t2.size > DUMP_T2_SAMPLE:
+        t2 = t2[np.sort(np.random.default_rng(0).choice(t2.size, DUMP_T2_SAMPLE, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("ccsd_iterate", [last["e_ccsd"], last["rms"]]), ("t1_diagnostic", [last["t1_diagnostic"]]),
+                    ("ccsd_t_sums", last["sums"]), ("t1", t1), ("t2_sample", t2)):
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+    log(f"outputs of the last timed step written to {out_dir}")
+
+
 # ------------------------------------------------------------------------------------------------ GPU arm
 def attach_comm(gpu, rank, world):
     import torch
@@ -226,9 +251,9 @@ def attach_comm(gpu, rank, world):
     gpu.comm_init(rank, world, bytes(uid.cpu().tolist()))
 
 
-def run_shape(args, rank, world, local, n, o, steps, warmup, e2e_first=False, want_hbm=True):
+def run_shape(args, rank, world, local, n, o, steps, warmup, e2e_first=False, want_hbm=True, dump_dir=None):
     """The hot path at one (nbf, nocc) shape: device-resident timed loop + e2e leg.  Returns the measurement dict
-    (rank 0) or None."""
+    (rank 0) or None.  dump_dir: see dump_outputs."""
     import torch
     import torch.distributed as dist
 
@@ -368,13 +393,14 @@ def run_shape(args, rank, world, local, n, o, steps, warmup, e2e_first=False, wa
     comp = {"ccsd": [], "diis": [], "t": []}
     gstat = {"ccsd": [0.0, 0.0, 0], "t": [0.0, 0.0, 0]}   # DMMA GEMM (ms, flop, launches) per stage of the timed region
     traj = []
+    last = {}
 
     def step(record):
         e, rms = gpu.ccsd_iterate()
         a = gpu.last_stage_ms()
         gpu.ccsd_diis()
         b = gpu.last_stage_ms()
-        gpu.ccsd_finalize()
+        t1_diag, _, _ = gpu.ccsd_finalize()
         if record:
             ms, fl, nl = gpu.gemm_stats()
             gstat["ccsd"][0] += ms; gstat["ccsd"][1] += fl; gstat["ccsd"][2] += nl
@@ -384,6 +410,7 @@ def run_shape(args, rank, world, local, n, o, steps, warmup, e2e_first=False, wa
             ms, fl, nl = gpu.gemm_stats()
             gstat["t"][0] += ms; gstat["t"][1] += fl; gstat["t"][2] += nl
         traj.append([e, float(sums[0]), rms])
+        last.update(e_ccsd=e, rms=rms, t1_diagnostic=t1_diag, sums=sums)
         if record:
             comp["ccsd"].append(a); comp["diis"].append(b); comp["t"].append(c)
 
@@ -408,6 +435,8 @@ def run_shape(args, rank, world, local, n, o, steps, warmup, e2e_first=False, wa
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
     elapsed, wall = float(tt[0].item()), float(tt[1].item())
     value = elapsed / steps
+    if dump_dir and rank == 0:   # before the e2e leg, which starts the CCSD state afresh
+        dump_outputs(gpu, dump_dir, last)
 
     if not e2e_first:
         e2e_value = e2e_leg(steps)
@@ -517,7 +546,7 @@ def run_ours(args, rank, world, local):
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
     n, o = args.nbf, args.nocc
     v = n - o
-    m = run_shape(args, rank, world, local, n, o, args.steps, args.warmup)
+    m = run_shape(args, rank, world, local, n, o, args.steps, args.warmup, dump_dir=args.dump_outputs)
     line = None
     if rank == 0:
         cpu = None
@@ -611,7 +640,13 @@ def main():
                                                         "aligned GEMM), 1 the (T) batches only, 0 cp.async kernels only")
     ap.add_argument("--dist-chunks", type=int, default=0, help="dist_overlap_chunks of the sharded CCSD GEMMs (0: library default)")
     ap.add_argument("--workload", default=None, help="sample_data molecule run: n2 | f2 | h2o | h2o-spinorb")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.workload or args.impl != "ours"):
+        ap.error("--dump-outputs applies to the GPU arm at the synthetic shape only")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))

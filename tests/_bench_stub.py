@@ -79,7 +79,10 @@ class FakeGpu:
     def ccsd_finalize(self, want_cr=False, want_amplitudes=False, out=None):
         if out is not None:
             assert out[0].size == self.o * self.v and out[1].size == self.o * self.o * self.v * self.v
-        return 0.01, None, None
+        if want_amplitudes:
+            t2 = np.linspace(-1e-3, 1e-3, (self.o * self.v) ** 2).reshape((self.o, self.o, self.v, self.v), order="F")
+            return 0.01 * self.iter, np.full((self.o, self.v), 1e-4 * self.iter), t2
+        return 0.01 * self.iter, None, None
     def ccsd_t_spatial(self, paren, renorm, cr): return np.array([-1e-3, -1e-3, 0, 0, 0, 0.0]), 0.0
     def set_partition(self, rank, nranks): self.partition = (rank, nranks)
 

@@ -7,6 +7,8 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 STUB = os.path.join(ROOT, "tests", "_bench_stub.py")
 KEYS = ["metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling", "vs_baseline",
@@ -88,6 +90,44 @@ def test_parity_block_uses_the_cpu_pins_and_the_pin_file_is_self_consistent():
                 "e_T_vs_cpu_first_steps", "e_ccsd_max_over_steps", "e_T_max_over_steps"):
         assert key in d["ok"]["abs_diff"], key
     assert d["bad"]["ok"] is False and d["bad"]["abs_diff"]["e_T_step1_vs_cpu_oracle"] > 1e-9
+
+
+def test_dump_outputs_writes_the_last_timed_step_and_steps_sets_the_step_count(tmp_path):
+    """--dump-outputs DIR: float64 .npy files of what the last timed step returned, identical from run to run; the fake
+    engine's energy and T1 diagnostic count the iterations since ccsd_init, so they show that exactly W + K steps ran
+    before the dump.  At nbf=100/nocc=12 T2 (1115136 elements) is larger than the sample: the fake engine's T2 holds
+    ascending values in column-major order, so the sample must be DUMP_T2_SAMPLE of them, distinct and ascending."""
+    names = {"ccsd_iterate.npy", "t1_diagnostic.npy", "ccsd_t_sums.npy", "t1.npy", "t2_sample.npy"}
+    runs = {}
+    for tag, steps, n, o in (("a", 2, 36, 4), ("b", 2, 36, 4), ("c", 5, 36, 4), ("d", 1, 100, 12), ("e", 1, 100, 12)):
+        out = tmp_path / tag
+        d = _run([sys.executable, STUB, "--gpus", "1", "--steps", str(steps), "--warmup", "1", "--nbf", str(n), "--nocc",
+                  str(o), "--no-cpu", "--target", "0", "--dump-outputs", str(out)], {})
+        assert d["steps"] == steps and set(os.listdir(out)) == names
+        arrs = {nm: np.load(out / nm) for nm in names}
+        assert all(a.dtype == np.float64 for a in arrs.values())
+        assert sum(a.nbytes for a in arrs.values()) <= 64 << 20
+        assert arrs["ccsd_t_sums.npy"].shape == (6,) and arrs["t1.npy"].shape == (o, n - o)
+        e, rms = arrs["ccsd_iterate.npy"]
+        assert e == d["energies"]["e_ccsd"] and rms == d["energies"]["rms"]
+        assert e == -0.1 - 0.01 / (1 + steps)                      # warm-up + timed iterations
+        assert arrs["t1_diagnostic.npy"].tolist() == [0.01 * (1 + steps)]
+        size = (o * (n - o)) ** 2
+        t2 = arrs["t2_sample.npy"]
+        if n == 36:
+            assert t2.size == size                                 # smaller than the sample: kept whole
+        else:
+            assert size > 1 << 20 and t2.size == 1 << 20            # bench.DUMP_T2_SAMPLE
+            full = np.linspace(-1e-3, 1e-3, size)
+            pos = np.rint((t2 + 1e-3) / 2e-3 * (size - 1)).astype(np.int64)
+            assert np.all(np.diff(pos) > 0) and np.array_equal(full[pos], t2)
+        runs[tag] = arrs
+    for a, b in (("a", "b"), ("d", "e")):
+        for nm in names:
+            assert np.array_equal(runs[a][nm], runs[b][nm]), (a, b, nm)
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], cwd=ROOT, capture_output=True,
+                       text=True, timeout=120)
+    assert r.returncode != 0 and "--steps" in r.stderr
 
 
 def test_per_triple_check_of_the_target_leg_is_attached_and_cannot_take_the_line_down(tmp_path):

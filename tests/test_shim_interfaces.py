@@ -5,18 +5,19 @@ shim/afesp_gpu.f90 is delivered as source only, so what CAN be verified without 
     arguments, each passed the way the C prototype expects (by value / by reference) and with the matching C type;
   * the shim covers every export of the header;
   * free-form source limits (132 columns, continuation markers) hold;
-  * every component of the reference's derived types the wrappers touch (sys%..., int_store%...) and every module
-    entity they import exists in the reference's sources (only where /root/reference is present: this container).
+  * every component of the reference's derived types the wrappers touch (sys%..., int_store%...), every module entity
+    they import and every printed line they keep exists in the reference's sources, as recorded in
+    tests/golden/reference_src.json (tests/golden/make_reference_src.py); the printed lines also appear in the outputs
+    the reference shipped (tests/golden/*_out.txt).
 """
+import json
 import os
 import re
-
-import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 SHIM = os.path.join(ROOT, "shim", "afesp_gpu.f90")
 HEADER = os.path.join(ROOT, "include", "afesp_gpu.h")
-REF_SRC = "/root/reference/src"
+GOLDEN = os.path.join(ROOT, "tests", "golden")
 
 
 # ------------------------------------------------------------------------------------------------ C prototypes
@@ -160,34 +161,31 @@ def test_wrappers_check_every_status():
     assert re.search(r"call check\(rc,", joined), "the kept status rc is never checked"
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_SRC), reason="reference sources only exist in the build container")
 def test_wrappers_only_touch_entities_the_reference_defines():
     shim = open(SHIM).read()
-    system = open(os.path.join(REF_SRC, "system.f90")).read().lower()
-    integrals = open(os.path.join(REF_SRC, "integrals.f90")).read().lower()
-    type_body = system.split("type system_t", 1)[1].split("end type", 1)[0]
+    ref = json.load(open(os.path.join(GOLDEN, "reference_src.json")))
     for comp in sorted(set(re.findall(r"\bsys%(\w+)", shim))):
-        assert re.search(r"\b%s\b" % comp.lower(), type_body), f"system_t has no component {comp}"
-    store_body = integrals.split("type int_store_t", 1)[1].split("end type", 1)[0]
+        assert comp.lower() in ref["system_t"], f"system_t has no component {comp}"
     for comp in sorted(set(re.findall(r"\bint_store%(\w+)", shim))):
-        assert re.search(r"\b%s\b" % comp.lower(), store_body), f"int_store_t has no component {comp}"
+        assert comp.lower() in ref["int_store_t"], f"int_store_t has no component {comp}"
     # module entities imported with `use <module>, only:`
     for mod, names in re.findall(r"use (\w+), only: ([\w, =>]+)", shim):
         if mod in ("iso_c_binding", "iso_fortran_env"):
             continue
-        src = open(os.path.join(REF_SRC, {"const": "const.F90"}.get(mod, mod + ".f90"))).read().lower()
         for nm in [x.split("=>")[-1].strip() for x in names.split(",")]:
-            assert re.search(r"\b%s\b" % nm.lower(), src), f"module {mod} has no entity {nm}"
+            assert nm.lower() in ref["modules"].get(mod, []), f"module {mod} has no entity {nm}"
     # the printed lines the wrappers keep are the reference's own format strings
-    ccsd = open(os.path.join(REF_SRC, "ccsd.f90")).read()
-    mp2 = open(os.path.join(REF_SRC, "mp2.f90")).read()
-    for text in ["Performing AO to MO ERI transformation...", "Calculating MP2 energy...",
-                 "MP2 correlation energy (Hartree):"]:
-        assert text in shim and text in mp2, text
-    for text in ["Convergence reached within tolerance.", "Final CCSD Energy (Hartree):", "T1 diagnostic:",
-                 "Forming antisymmetrised spinorbital ERIs...",
-                 "Checking that the permuational symmetry of the antisymmetrised integrals hold...",
-                 "Permutational symmetry of antisymmetrised integrals does not hold",
-                 "Unrestricted CCSD(T) correlation energy (Hartree):",
-                 "(1X, I9, 3X, F15.12, 3X, F15.12, 3X, F15.12, 3X, F8.6)"]:
-        assert text in shim and text in ccsd, text
+    printed = {"mp2.f90": ["Performing AO to MO ERI transformation...", "Calculating MP2 energy...",
+                           "MP2 correlation energy (Hartree):"],
+               "ccsd.f90": ["Convergence reached within tolerance.", "Final CCSD Energy (Hartree):", "T1 diagnostic:",
+                            "Forming antisymmetrised spinorbital ERIs...",
+                            "Checking that the permuational symmetry of the antisymmetrised integrals hold...",
+                            "Unrestricted CCSD(T) correlation energy (Hartree):"]}
+    kept = {"ccsd.f90": ["Permutational symmetry of antisymmetrised integrals does not hold",   # error path
+                         "(1X, I9, 3X, F15.12, 3X, F15.12, 3X, F15.12, 3X, F8.6)"]}         # iteration-table format
+    shipped = "".join(open(os.path.join(GOLDEN, f)).read() for f in sorted(os.listdir(GOLDEN)) if f.endswith("_out.txt"))
+    for fname in ("mp2.f90", "ccsd.f90"):
+        for text in printed[fname] + kept.get(fname, []):
+            assert text in shim and text in ref["strings"][fname], (fname, text)
+        for text in printed[fname]:
+            assert text in shipped, text
