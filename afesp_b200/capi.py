@@ -109,6 +109,7 @@ class AfespGpu:
         self.n = 0
         self.o = 0
         self.v = 0
+        self.frozen_core = 0   # option "frozen_core" as last set; ccsd_init sizes the amplitudes from it
 
     # -- plumbing
     def _check(self, fn, rc):
@@ -134,6 +135,8 @@ class AfespGpu:
 
     def set_option(self, key, value):
         self._check("set_option", self.lib.afesp_gpu_set_option(self.h, key.encode(), float(value)))
+        if key == "frozen_core":
+            self.frozen_core = int(value)
 
     def counters(self):
         n = C.c_longlong(0)
@@ -199,10 +202,11 @@ class AfespGpu:
         e1, r = C.c_double(0), C.c_double(0)
         self._check("ccsd_init", self.lib.afesp_gpu_ccsd_init(self.h, int(nocc), int(bool(restricted)), _ptr(e),
                                                               int(diis_n), C.byref(e1), C.byref(r)))
+        nact = int(nocc) - self.frozen_core   # t1 / t2 cover the active occupied orbitals only
         if restricted:
-            self.o, self.v = int(nocc), self.n - int(nocc)
+            self.o, self.v = nact, self.n - int(nocc)
         else:
-            self.o, self.v = 2 * int(nocc), 2 * (self.n - int(nocc))
+            self.o, self.v = 2 * nact, 2 * (self.n - int(nocc))
         return e1.value, r.value
 
     def ccsd_init_info(self):

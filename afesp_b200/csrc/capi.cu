@@ -80,6 +80,7 @@ struct Handle {
   CCState s;
   DBuf eri_ao, coeff;
   int n_ao = 0;
+  int frozen_core = 0;   // option "frozen_core": read by mp2_energy and ccsd_init (which copies it into the CC state)
   std::string err;
   int rank = 0, nranks = 1;
   NcclComm comm = nullptr;
@@ -251,6 +252,11 @@ int afesp_gpu_set_option(afesp_handle hv, const char* key, double value) {
     else if (k == "triples_batch_bytes") o.triples_batch_bytes = (long long)value;
     else if (k == "finalize_keep_ccsd") o.finalize_keep_ccsd = value != 0.0;
     else if (k == "spinorb_symmetry_tol") o.spinorb_symmetry_tol = value;
+    else if (k == "frozen_core") {
+      AFESP_REQUIRE(value >= 0.0 && value == std::floor(value) && value < 1e9,
+                    "set_option: frozen_core must be a non-negative integer (number of frozen doubly occupied orbitals)");
+      h.frozen_core = (int)value;
+    }
     else if (k == "gemm_timing") gemm_timing_enable(value != 0.0);
     else if (k == "gemm_force_config") gemm_force_config((int)value);
     else if (k == "gemm_tma_edge") gemm_tma_edge((int)value);
@@ -398,10 +404,12 @@ int afesp_gpu_mp2_energy(afesp_handle hv, int nocc, const double* eps, double* e
   return guarded(hv, [&](Handle& h) {
     AFESP_REQUIRE(h.s.n > 0 && h.s.eri_mo.p, "mp2_energy: no MO integrals on the device");
     AFESP_REQUIRE(nocc > 0 && nocc < h.s.n && e_mp2, "mp2_energy: bad arguments");
+    AFESP_REQUIRE(h.frozen_core < nocc, "mp2_energy: frozen_core (" + std::to_string(h.frozen_core) +
+                                            ") must be smaller than nocc (" + std::to_string(nocc) + ")");
     upload_eps(h, eps);
     if (h.s.red_out.n < 16) h.s.red_out.alloc(16);
     StageTimer tm(&h);
-    mp2_energy(h.s.eng, h.s.n, nocc, h.s.eri_mo.p, h.s.eps.p, h.s.red_out.p);
+    mp2_energy(h.s.eng, h.s.n, nocc, h.frozen_core, h.s.eri_mo.p, h.s.eps.p, h.s.red_out.p);
     tm.stop();
     AFESP_CUDA_CHECK(cudaMemcpy(e_mp2, h.s.red_out.p, 8, cudaMemcpyDeviceToHost));
   });
@@ -412,8 +420,11 @@ int afesp_gpu_ccsd_init(afesp_handle hv, int nocc, int restricted, const double*
   return guarded(hv, [&](Handle& h) {
     AFESP_REQUIRE(h.s.n > 0 && h.s.eri_mo.p, "ccsd_init: no MO integrals on the device");
     AFESP_REQUIRE(nocc > 0 && nocc < h.s.n, "ccsd_init: bad nocc");
+    AFESP_REQUIRE(h.frozen_core < nocc, "ccsd_init: frozen_core (" + std::to_string(h.frozen_core) +
+                                            ") must be smaller than nocc (" + std::to_string(nocc) + ")");
     upload_eps(h, eps);
     h.s.nocc_spatial = nocc;
+    h.s.nfrozen = h.frozen_core;
     {
       Trace tr(h.s.eng.stream);
       h.s.T.clear();
@@ -469,8 +480,8 @@ int afesp_gpu_ccsd_finalize(afesp_handle hv, int want_cr, double* t1_diag, doubl
     CCState& s = h.s;
     StageTimer tm(&h);
     if (t1_diag) {
-      // sqrt(sum t1^2)/sqrt(nel), nel = number of electrons (src/ccsd.f90:372)
-      *t1_diag = std::sqrt(cc_t1_norm2(s)) / std::sqrt((double)(2 * s.nocc_spatial));
+      // sqrt(sum t1^2)/sqrt(nel), nel = number of correlated electrons (src/ccsd.f90:372)
+      *t1_diag = std::sqrt(cc_t1_norm2(s)) / std::sqrt((double)(2 * (s.nocc_spatial - s.nfrozen)));
     }
     if (want_cr && !s.have_cr) {
       AFESP_REQUIRE(s.restricted, "CR intermediates exist only in the spin-free formulation");

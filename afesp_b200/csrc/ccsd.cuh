@@ -36,6 +36,7 @@ struct CCState {
   Engine eng;
   Options opt;
   int n = 0, nocc_spatial = 0;
+  int nfrozen = 0;   // frozen doubly occupied orbitals 0..nfrozen-1: the CC equations see orbitals nfrozen..n-1 only
   bool restricted = true;
   int o = 0, v = 0;  // occupied / virtual counts in the active formulation (spin-orbital counts when !restricted)
 

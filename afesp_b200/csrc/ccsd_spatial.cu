@@ -24,15 +24,16 @@ inline TView V(Tensor& t) { return t.view(); }
 }  // namespace
 
 void ccsd_spatial_init(CCState& s, int diis_n) {
-  const int n = s.n, o = s.nocc_spatial, v = n - o;
+  // active occupied orbitals start at nf (frozen core), virtual ones at nocc
+  const int n = s.n, nocc = s.nocc_spatial, nf = s.nfrozen, o = nocc - nf, v = n - nocc;
   s.restricted = true;
   s.o = o; s.v = v;
   AFESP_REQUIRE(o > 0 && v > 0, "ccsd init: need at least one occupied and one virtual orbital");
   Engine& e = s.eng;
   Trace tr(e.stream);
   s.eo.init({o}); s.ev.init({v});
-  AFESP_CUDA_CHECK(cudaMemcpyAsync(s.eo.p(), s.eps.p, o * 8, cudaMemcpyDeviceToDevice, e.stream));
-  AFESP_CUDA_CHECK(cudaMemcpyAsync(s.ev.p(), s.eps.p + o, v * 8, cudaMemcpyDeviceToDevice, e.stream));
+  AFESP_CUDA_CHECK(cudaMemcpyAsync(s.eo.p(), s.eps.p + nf, o * 8, cudaMemcpyDeviceToDevice, e.stream));
+  AFESP_CUDA_CHECK(cudaMemcpyAsync(s.ev.p(), s.eps.p + nocc, v * 8, cudaMemcpyDeviceToDevice, e.stream));
   // integral slices, physicist order (src/ccsd.f90:507-512)
   struct Sl { const char* name; char k[5]; };
   const Sl sl[] = {{"v_oovv", "oovv"}, {"v_ovov", "ovov"}, {"v_vvov", "vvov"},
@@ -41,7 +42,7 @@ void ccsd_spatial_init(CCState& s, int diis_n) {
     int lo[4], cnt[4];
     std::vector<int> dims;
     for (int d = 0; d < 4; ++d) {
-      lo[d] = x.k[d] == 'o' ? 0 : o;
+      lo[d] = x.k[d] == 'o' ? nf : nocc;
       cnt[d] = x.k[d] == 'o' ? o : v;
       dims.push_back(cnt[d]);
     }
@@ -65,10 +66,10 @@ void ccsd_spatial_init(CCState& s, int diis_n) {
     long long p0 = 0, p1 = Pp, m0 = 0, m1 = Pm;
     if (s.vpm_sharded) { d.col_range(Pp, d.rank, &p0, &p1); d.col_range(Pm, d.rank, &m0, &m1); }
     Tensor& Vp = s.make("V_plus", {(int)Pp, (int)std::max<long long>(p1 - p0, 1)});
-    build_vpm(e, Vp.p(), s.eri_mo.p, o, v, +1, p0, p1 - p0);
+    build_vpm(e, Vp.p(), s.eri_mo.p, nocc, v, +1, p0, p1 - p0);
     if (Pm > 0) {
       Tensor& Vm = s.make("V_minus", {(int)Pm, (int)std::max<long long>(m1 - m0, 1)});
-      build_vpm(e, Vm.p(), s.eri_mo.p, o, v, -1, m0, m1 - m0);
+      build_vpm(e, Vm.p(), s.eri_mo.p, nocc, v, -1, m0, m1 - m0);
     }
   }
 
@@ -289,11 +290,12 @@ void ccsd_spatial_cr_intermediates(CCState& s) {
     // the gathered slab in place), then a strided permute-add into Ivv(c,i,a0+a',b).
     const long long v3 = (long long)v * v * v;
     const int nb = (int)std::max<long long>(1, std::min<long long>(v, (4LL << 30) / (v3 * 8)));
+    const int nocc = s.nocc_spatial;   // first virtual orbital in the packed MO integrals
     Scratch slab(e.pool, (size_t)(v3 * nb)), y(e.pool, (size_t)((long long)o * v * v * nb));
     const long long ostr[4] = {1, v, (long long)v * o * v, (long long)v * o};   // out axes (c, i, b, a') inside Ivv
     for (int a0 = 0; a0 < v; a0 += nb) {
       const int cb = std::min(nb, v - a0);
-      const int lo4[4] = {o, o, o, o + a0}, cnt4[4] = {v, v, v, cb};
+      const int lo4[4] = {nocc, nocc, nocc, nocc + a0}, cnt4[4] = {v, v, v, cb};
       slice_phys(e, slab.p, s.eri_mo.p, lo4, cnt4);                       // slab(e,c,b,a')
       TView SL(slab.p, {v, v, v, cb}), Y(y.p, {o, v, v, cb});
       einsum(e, "ie,ecba->icba", 1.0, V(t1), SL, 0.0, Y);

@@ -15,7 +15,9 @@ inline TView V(Tensor& t) { return t.view(); }
 
 void ccsd_spinorb_init(CCState& s, int diis_n) {
   const int n = s.n;
-  const int o = 2 * s.nocc_spatial, v = 2 * n - o;
+  // active occupied spin-orbitals start at 2 nfrozen (frozen core), virtual ones at 2 nocc
+  const int olo = 2 * s.nfrozen, vlo = 2 * s.nocc_spatial;
+  const int o = vlo - olo, v = 2 * n - vlo;
   s.restricted = false;
   s.o = o; s.v = v;
   AFESP_REQUIRE(o > 0 && v > 0, "ccsd init: need at least one occupied and one virtual orbital");
@@ -24,8 +26,8 @@ void ccsd_spinorb_init(CCState& s, int diis_n) {
   std::vector<double> es(2 * n);
   for (int p = 0; p < n; ++p) es[2 * p] = es[2 * p + 1] = s.eps_host[p];
   s.eo.init({o}); s.ev.init({v});
-  AFESP_CUDA_CHECK(cudaMemcpyAsync(s.eo.p(), es.data(), o * 8, cudaMemcpyHostToDevice, e.stream));
-  AFESP_CUDA_CHECK(cudaMemcpyAsync(s.ev.p(), es.data() + o, v * 8, cudaMemcpyHostToDevice, e.stream));
+  AFESP_CUDA_CHECK(cudaMemcpyAsync(s.eo.p(), es.data() + olo, o * 8, cudaMemcpyHostToDevice, e.stream));
+  AFESP_CUDA_CHECK(cudaMemcpyAsync(s.ev.p(), es.data() + vlo, v * 8, cudaMemcpyHostToDevice, e.stream));
   AFESP_CUDA_CHECK(cudaStreamSynchronize(e.stream));
   // nine slices of <pq||rs> (src/ccsd.f90:182-194), gathered straight from the packed MO integrals: the (2n)^4
   // tensor of :108 is never formed.
@@ -36,7 +38,7 @@ void ccsd_spinorb_init(CCState& s, int diis_n) {
     int lo[4], cnt[4];
     std::vector<int> dims;
     for (int d = 0; d < 4; ++d) {
-      lo[d] = nm[d] == 'o' ? 0 : o;
+      lo[d] = nm[d] == 'o' ? olo : vlo;
       cnt[d] = nm[d] == 'o' ? o : v;
       dims.push_back(cnt[d]);
     }
@@ -45,9 +47,9 @@ void ccsd_spinorb_init(CCState& s, int diis_n) {
   }
   AFESP_CUDA_CHECK(cudaEventRecord(ev[1], e.stream));
   // the reference's run-time assertion on <pq||rs> (src/ccsd.f90:150-167): same index set, same four identities, same
-  // threshold (depsilon); a violation aborts the calculation with the reference's message
+  // threshold (depsilon), over the active spin-orbitals; a violation aborts the calculation with the reference's message
   if (s.red_out.n < 16) s.red_out.alloc(16);
-  spinorb_symmetry_error(e, n, s.eri_mo.p, s.red_out.p);
+  spinorb_symmetry_error(e, n, olo, s.eri_mo.p, s.red_out.p);
   AFESP_CUDA_CHECK(cudaEventRecord(ev[2], e.stream));
   AFESP_CUDA_CHECK(cudaMemcpyAsync(&s.sym_err, s.red_out.p, 8, cudaMemcpyDeviceToHost, e.stream));
   AFESP_CUDA_CHECK(cudaStreamSynchronize(e.stream));

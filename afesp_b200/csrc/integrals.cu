@@ -93,10 +93,11 @@ __global__ void k_pack_pairs(double* __restrict__ D, const double* __restrict__ 
   }
 }
 
+// i, j run over the active occupied orbitals [k, o), a, b over the virtuals [o, n)
 __global__ void __launch_bounds__(256) k_mp2(const double* __restrict__ g, const double* __restrict__ eps, int n, int o,
-                                              double* __restrict__ partials) {
-  const int v = n - o;
-  const long long total = (long long)o * o * v * v;
+                                              int k, double* __restrict__ partials) {
+  const int v = n - o, oa = o - k;
+  const long long total = (long long)oa * oa * v * v;
   double acc = 0.0;
   for (long long idx = blockIdx.x * (long long)blockDim.x + threadIdx.x; idx < total;
        idx += (long long)gridDim.x * blockDim.x) {
@@ -104,7 +105,7 @@ __global__ void __launch_bounds__(256) k_mp2(const double* __restrict__ g, const
     long long t = idx / v;
     int a = (int)(t % v) + o;
     t /= v;
-    int j = (int)(t % o), i = (int)(t / o);
+    int j = (int)(t % oa) + k, i = (int)(t / oa) + k;
     long long ia = tri(i, a), jb = tri(j, b), ib = tri(i, b), ja = tri(j, a);
     double iajb = g[tri(ia, jb)];
     acc += iajb * (2.0 * iajb - g[tri(ib, ja)]) / (eps[i] + eps[j] - eps[a] - eps[b]);
@@ -163,16 +164,17 @@ __device__ __forceinline__ double asym_spinorb(const double* __restrict__ g, int
   if ((P & 1) == (S & 1) && (Q & 1) == (R & 1)) val -= g[tri(tri(p, s), tri(q, r))];
   return val;
 }
-__global__ void k_spinorb_symmetry(const double* __restrict__ g, int n2, double* __restrict__ partials) {
+// The box is the spin-orbitals [lo, lo + n2): lo = 2k when k core orbitals are frozen.
+__global__ void k_spinorb_symmetry(const double* __restrict__ g, int lo, int n2, double* __restrict__ partials) {
   const long long total = (long long)n2 * n2 * n2 * n2;
   double err = 0.0;
   for (long long idx = blockIdx.x * (long long)blockDim.x + threadIdx.x; idx < total;
        idx += (long long)gridDim.x * blockDim.x) {
     long long t = idx;
-    const int s = (int)(t % n2); t /= n2;
-    const int r = (int)(t % n2); t /= n2;
-    const int q = (int)(t % n2);
-    const int p = (int)(t / n2);
+    const int s = (int)(t % n2) + lo; t /= n2;
+    const int r = (int)(t % n2) + lo; t /= n2;
+    const int q = (int)(t % n2) + lo;
+    const int p = (int)(t / n2) + lo;
     if (q > p || r > p || s > r) continue;
     const double x = asym_spinorb(g, p, q, r, s);
     err += fabs(x + asym_spinorb(g, p, q, s, r)) + fabs(x - asym_spinorb(g, r, s, p, q)) +
@@ -192,8 +194,8 @@ __global__ void k_spinorb_symmetry(const double* __restrict__ g, int n2, double*
 // (+/-)-symmetrised virtual-pair integrals for the particle-particle ladder:
 //   Vp(ef, ab) = <ef|ab> + <ef|ba>,  e<=f, a<=b   (P+ = v(v+1)/2 pairs, pair(a,b) = b(b+1)/2 + a)
 //   Vm(ef, ab) = <ef|ab> - <ef|ba>,  e<f,  a<b    (P- = v(v-1)/2 pairs, pair(a,b) = b(b-1)/2 + a)
-// <ef|ab> = (ea|fb), virtual indices offset by nocc in the packed MO array.
-__global__ void k_build_vpm(double* __restrict__ V, const double* __restrict__ g, int o, int v, int sign,
+// <ef|ab> = (ea|fb), virtual indices offset by voff (= nocc) in the packed MO array.
+__global__ void k_build_vpm(double* __restrict__ V, const double* __restrict__ g, int voff, int v, int sign,
                             long long col0, long long ncols) {
   const long long P = sign > 0 ? (long long)v * (v + 1) / 2 : (long long)v * (v - 1) / 2;
   const long long total = P * ncols;
@@ -220,7 +222,7 @@ __global__ void k_build_vpm(double* __restrict__ V, const double* __restrict__ g
       while ((b + 1) * b / 2 <= ab) ++b;
       a = ab - b * (b - 1) / 2;
     }
-    const long long E = e + o, F = f + o, A = a + o, B = b + o;
+    const long long E = e + voff, F = f + voff, A = a + voff, B = b + voff;
     const double x = g[tri(tri(E, A), tri(F, B))];   // <ef|ab>
     const double y = g[tri(tri(E, B), tri(F, A))];   // <ef|ba>
     V[idx] = sign > 0 ? x + y : x - y;
@@ -393,31 +395,31 @@ void ao2mo_packed(Engine& e, int n, const double* eri_ao, const double* C, doubl
   d.exchange(eri_mo, ranges, e.stream);
 }
 
-void mp2_energy(Engine& e, int n, int nocc, const double* eri_mo, const double* eps, double* out_dev) {
-  const long long total = (long long)nocc * nocc * (n - nocc) * (n - nocc);
+void mp2_energy(Engine& e, int n, int nocc, int nfrozen, const double* eri_mo, const double* eps, double* out_dev) {
+  const long long total = (long long)(nocc - nfrozen) * (nocc - nfrozen) * (n - nocc) * (n - nocc);
   int nb = std::min(grid_for(total), 1024);
   double* part = reduce_scratch(e, nb);
-  k_mp2<<<nb, 256, 0, e.stream>>>(eri_mo, eps, n, nocc, part);
+  k_mp2<<<nb, 256, 0, e.stream>>>(eri_mo, eps, n, nocc, nfrozen, part);
   count_launch();
   finish_partials(e, part, nb, 1, out_dev);
 }
 
-void spinorb_symmetry_error(Engine& e, int n, const double* eri_mo, double* out_dev) {
-  const int n2 = 2 * n;
+void spinorb_symmetry_error(Engine& e, int n, int lo, const double* eri_mo, double* out_dev) {
+  const int n2 = 2 * n - lo;
   const long long total = (long long)n2 * n2 * n2 * n2;
   const int nb = std::min(grid_for(total), 148 * 8);
   double* part = reduce_scratch(e, nb);
-  k_spinorb_symmetry<<<nb, 256, 0, e.stream>>>(eri_mo, n2, part);
+  k_spinorb_symmetry<<<nb, 256, 0, e.stream>>>(eri_mo, lo, n2, part);
   count_launch();
   AFESP_CUDA_CHECK(cudaGetLastError());
   finish_partials(e, part, nb, 1, out_dev);
 }
 
-void build_vpm(Engine& e, double* V, const double* eri_mo, int o, int v, int sign, long long col0, long long ncols) {
+void build_vpm(Engine& e, double* V, const double* eri_mo, int voff, int v, int sign, long long col0, long long ncols) {
   const long long P = sign > 0 ? (long long)v * (v + 1) / 2 : (long long)v * (v - 1) / 2;
   if (ncols < 0) ncols = P - col0;
   if (P == 0 || ncols <= 0) return;
-  k_build_vpm<<<grid_for(P * ncols), 256, 0, e.stream>>>(V, eri_mo, o, v, sign, col0, ncols);
+  k_build_vpm<<<grid_for(P * ncols), 256, 0, e.stream>>>(V, eri_mo, voff, v, sign, col0, ncols);
   count_launch();
 }
 

@@ -447,14 +447,17 @@ void triples_spatial(CCState& s, bool paren, bool renorm, bool comp_renorm, int 
   // K-concatenated GEMM operands (work arrays come from the engine's pool: cudaFree of GB-sized blocks is slow).
   // With the hole term written in the layout (c,b,a) it lands in the buffer of the permutation (r,q,p) as
   //     C_pqr(x,(y,z)) = sum_d t2(p,q,x,d) v_vovv(d,r,y,z) - sum_l v_ovoo(l,x,q,p) t2(l,r,y,z)
-  // i.e. ONE product of depth K = v + o = nbf per permutation:
+  // i.e. ONE product of depth K = v + o (= nbf without frozen core) per permutation:
   //     Acat(x, [d | l]; p,q) = [ t2(p,q,x,d) | -v_oovo(p,q,x,l) ]            (v x n) for each occupied pair
   //     Bcat([d | l], (y,z); r) = [ v_vvov(z,y,r,d) ; t2(l,r,y,z) ]           (n x v^2) for each occupied index
   //     BcatT(k, (y,z); r)      = Bcat(k, (z,y); r)
   // (the reference's reshapes at :2056-2066, re-aimed at GEMM blocks).  M3 uses I_ooov_pp / I_vovv_pp instead (:2188-2193).
   // The two permutations with the same first label are then one dual-segment GEMM (see the file header):
   //     Y_s(x,(u,w); i,j,k) = Acat(x,.; P0,P1) Bcat(.,(u,w); P2) + Acat(x,.; P0,P2) BcatT(.,(u,w); P1),  (P0,P1,P2) = p_s(i,j,k)
-  const int n = v + o;
+  // K = v + o is also the leading dimension of Bcat and the block stride of both operands.  With v even and o odd (e.g. an
+  // odd number of frozen core orbitals) one zero column of Acat and one zero row of Bcat / BcatT make K even, so the
+  // batches keep the 16-byte-aligned (TMA) kernel; the zero terms change only the grouping of the last k-tile.
+  const int n = v + o + ((v % 2 == 0 && o % 2 == 1) ? 1 : 0);
   const size_t n_acat = (size_t)v * n * o * o, n_bcat = (size_t)n * v2 * o;
   Scratch sAcat(e.pool, n_acat + 16), sBcat(e.pool, n_bcat + 16), sBcatT(e.pool, n_bcat + 16);  // +16: TMA boxes over-read the last 16-row chunk
   std::unique_ptr<Scratch> sAcatM, sBcatM, sBcatMT;
@@ -474,6 +477,13 @@ void triples_spatial(CCState& s, bool paren, bool renorm, bool comp_renorm, int 
   put(s.t2.view(), "lryz", "lyzr", 1.0, sBcat.p + v, b_str);
   put(s.get("v_vvov").view(), "yzrd", "dyzr", 1.0, sBcatT.p, b_str);
   put(s.t2.view(), "lrzy", "lyzr", 1.0, sBcatT.p + v, b_str);
+  auto zero_pad = [&](double* Acat, double* Bcat, double* BcatT) {   // pool scratch is not zeroed
+    if (n == v + o) return;
+    AFESP_CUDA_CHECK(cudaMemset2DAsync(Acat + (size_t)v * (v + o), (size_t)v * n * 8, 0, (size_t)v * 8, (size_t)o * o, st));
+    AFESP_CUDA_CHECK(cudaMemset2DAsync(Bcat + (v + o), (size_t)n * 8, 0, 8, (size_t)v2 * o, st));
+    AFESP_CUDA_CHECK(cudaMemset2DAsync(BcatT + (v + o), (size_t)n * 8, 0, 8, (size_t)v2 * o, st));
+  };
+  zero_pad(sAcat.p, sBcat.p, sBcatT.p);
   if (do_m) {
     sAcatM.reset(new Scratch(e.pool, n_acat + 16)); sBcatM.reset(new Scratch(e.pool, n_bcat + 16));
     sBcatMT.reset(new Scratch(e.pool, n_bcat + 16));
@@ -483,6 +493,7 @@ void triples_spatial(CCState& s, bool paren, bool renorm, bool comp_renorm, int 
     put(s.t2.view(), "lryz", "lyzr", 1.0, sBcatM->p + v, b_str);
     put(s.get("I_vovv_pp").view(), "drzy", "dyzr", 1.0, sBcatMT->p, b_str);
     put(s.t2.view(), "lrzy", "lyzr", 1.0, sBcatMT->p + v, b_str);
+    zero_pad(sAcatM->p, sBcatM->p, sBcatMT->p);
   }
 
   std::vector<TripleDesc> tri = my_triples(o, s.opt.triples_ijk_symmetry, false, rank, nranks);
@@ -534,7 +545,7 @@ void triples_spatial(CCState& s, bool paren, bool renorm, bool comp_renorm, int 
   Scratch tiles_d(e.pool, (tiles_h.size() + 1) / 2 + 1);
   AFESP_CUDA_CHECK(cudaMemcpyAsync(tiles_d.p, tiles_h.data(), tiles_h.size() * sizeof(int), cudaMemcpyHostToDevice, st));
   static_assert(sizeof(TripleDesc) == 40, "TripleDesc layout");
-  const bool al16 = (v % 2 == 0) && (o % 2 == 0);
+  const bool al16 = (v % 2 == 0) && (n % 2 == 0);
 
   // Launch tables of ALL batches, built on the host and uploaded once (no per-batch synchronisation): the triple
   // descriptors, and per GEMM block the (A pair, B index) of both K segments as block indices (TMA gather form) and as

@@ -53,6 +53,7 @@ class ElsInput:
     write_fcidump: bool = False
     scf_read_guess: bool = False
     scf_write_guess: bool = False
+    frozen_core: int = 0               # frozen doubly occupied orbitals (extension of the namelist; 0 = all-electron)
     nbasis: int = 0
     nel: int = 0
     e_nuc: float = 0.0
@@ -90,7 +91,8 @@ def pair_index(i, j):
 
 NAMELIST_KEYS = {"calc_type": str, "scf_e_tol": float, "scf_d_tol": float, "ccsd_e_tol": float, "ccsd_t_tol": float,
                  "scf_diis_n_errmat": int, "ccsd_diis_n_errmat": int, "scf_maxiter": int, "ccsd_maxiter": int,
-                 "write_fcidump": bool, "scf_read_guess": bool, "scf_write_guess": bool}   # src/system.f90:96-97
+                 "write_fcidump": bool, "scf_read_guess": bool, "scf_write_guess": bool,   # src/system.f90:96-97
+                 "frozen_core": int}
 
 
 def parse_namelist(text):
@@ -225,6 +227,13 @@ def set_geometry(inp: ElsInput, charges, xyz):
         for i in range(j):
             e += z[i] * z[j] / np.linalg.norm(xyz[i] - xyz[j])
     inp.e_nuc = e
+
+
+def check_frozen_core(inp: ElsInput):
+    """frozen_core must leave at least one doubly occupied orbital active (same text as host/els_host.cpp)."""
+    nocc = inp.nel // 2
+    if not 0 <= inp.frozen_core < nocc:
+        raise ValueError("system::read_system_in: frozen_core = %d is outside 0..%d (nocc - 1)!" % (inp.frozen_core, nocc - 1))
 
 
 def _unpack(packed, n):
@@ -433,6 +442,7 @@ def run(inp: ElsInput, gpu: AfespGpu | None = None, device: int = 0, verbose: bo
     With `workdir` the files the reference writes into its run directory are written there too: guess_out.dat
     (scf_write_guess) and FCIDUMP (write_fcidump)."""
     level, restricted, paren, renorm, comp_renorm = CALC_TYPES[inp.calc_type]
+    check_frozen_core(inp)
     out = io.StringIO()
     res = ElsResult(e_nuc=inp.e_nuc)
     t_glob = time.perf_counter()
@@ -455,6 +465,8 @@ def run(inp: ElsInput, gpu: AfespGpu | None = None, device: int = 0, verbose: bo
         gpu = gpu or AfespGpu(device)
         try:
             nocc = inp.nel // 2
+            if inp.frozen_core > 0:   # MP2, CCSD and the triples correlate orbitals frozen_core.. only
+                gpu.set_option("frozen_core", inp.frozen_core)
             t0 = time.perf_counter()
             out.write(" ----------\n MP2\n ----------\n Performing AO to MO ERI transformation...\n")
             gpu.ao2mo(inp.nbasis, inp.eri, C_mo, want_result=False)
@@ -565,8 +577,10 @@ def header_block(inp: ElsInput, when=None) -> str:
          " Reading two-body integrals...", " Done reading integrals!",
          " " + "-" * 20, " System information", " " + "-" * 20,
          " Number of electrons: %d" % inp.nel, " Number of basis functions: %d" % inp.nbasis,
-         " Number of occupied orbitals: %d" % nocc_print, " Number of virtual orbitals: %d" % nvirt_print,
-         " E_nuc: " + _es_f(inp.e_nuc, 15, 8),
+         " Number of occupied orbitals: %d" % nocc_print, " Number of virtual orbitals: %d" % nvirt_print]
+    if inp.frozen_core > 0:
+        L.append(" Number of frozen core orbitals: %d" % inp.frozen_core)
+    L += [" E_nuc: " + _es_f(inp.e_nuc, 15, 8),
          " scf_e_tol: " + _es_f(inp.scf_e_tol, 8, 2), " scf_d_tol: " + _es_f(inp.scf_d_tol, 8, 2),
          " ccsd_e_tol: " + _es_f(inp.ccsd_e_tol, 8, 2), " ccsd_t_tol: " + _es_f(inp.ccsd_t_tol, 8, 2),
          " Number of SCF DIIS error matrices: %d" % inp.scf_diis_n_errmat,

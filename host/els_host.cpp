@@ -62,6 +62,7 @@ struct Sys {
   double scf_e_tol = 1e-6, scf_d_tol = 1e-6, ccsd_e_tol = 1e-6, ccsd_t_tol = 1e-6;
   int scf_diis_n_errmat = 6, ccsd_diis_n_errmat = 8, scf_maxiter = 50, ccsd_maxiter = 50;
   bool write_fcidump = false, scf_read_guess = false, scf_write_guess = false;
+  int frozen_core = 0;   // frozen doubly occupied orbitals (extension of the namelist; 0 = all-electron)
   int nbasis = 0, nel = 0;
   double e_nuc = 0.0;
   std::vector<double> ovlp, hcore, eri, guess;  // n x n row-major (symmetric), packed ERIs
@@ -190,6 +191,7 @@ void read_system_in(Sys& s) {
     else if (k == "write_fcidump") s.write_fcidump = as_bool(v);
     else if (k == "scf_read_guess") s.scf_read_guess = as_bool(v);
     else if (k == "scf_write_guess") s.scf_write_guess = as_bool(v);
+    else if (k == "frozen_core") s.frozen_core = as_int(v);
     else bad();
   }
   set_calc_type(s);
@@ -583,14 +585,19 @@ int main(int argc, char** argv) {
   std::printf(" Done reading integrals!\n");
   read_geometry_in(s);
   const int n = s.nbasis, nocc = s.nel / 2;
+  if (s.frozen_core < 0 || s.frozen_core >= nocc)   // at least one doubly occupied orbital stays active
+    fail("system::read_system_in", "frozen_core = " + std::to_string(s.frozen_core) + " is outside 0.." +
+                                       std::to_string(nocc - 1) + " (nocc - 1)!");
   // print_sys_info (src/integrals.f90:223-249)
   std::printf(" %s\n System information\n %s\n", bar(20, '-').c_str(), bar(20, '-').c_str());
   std::printf(" Number of electrons: %d\n Number of basis functions: %d\n Number of occupied orbitals: %d\n"
-              " Number of virtual orbitals: %d\n E_nuc: %15.8E\n scf_e_tol: %8.2E\n scf_d_tol: %8.2E\n ccsd_e_tol: %8.2E\n"
+              " Number of virtual orbitals: %d\n",
+              s.nel, n, s.restricted ? nocc : s.nel, s.restricted ? n - nocc : 2 * (n - nocc));   // src/geometry.f90:40-46
+  if (s.frozen_core > 0) std::printf(" Number of frozen core orbitals: %d\n", s.frozen_core);
+  std::printf(" E_nuc: %15.8E\n scf_e_tol: %8.2E\n scf_d_tol: %8.2E\n ccsd_e_tol: %8.2E\n"
               " ccsd_t_tol: %8.2E\n Number of SCF DIIS error matrices: %d\n Number of CCSD DIIS error matrices: %d\n"
               " Maximum number of SCF iterations: %d\n Maximum number of CCSD iterations: %d\n"
               " Printing out the input file...\n%s\n",
-              s.nel, n, s.restricted ? nocc : s.nel, s.restricted ? n - nocc : 2 * (n - nocc),   // src/geometry.f90:40-46
               s.e_nuc, s.scf_e_tol, s.scf_d_tol, s.ccsd_e_tol, s.ccsd_t_tol,
               s.scf_diis_n_errmat, s.ccsd_diis_n_errmat, s.scf_maxiter, s.ccsd_maxiter, bar(30, '-').c_str());
   {
@@ -647,6 +654,8 @@ int main(int argc, char** argv) {
         pos = end + 1;
       }
     }
+    // MP2, CCSD and the triples correlate orbitals frozen_core.. only
+    if (s.frozen_core > 0) check("set_option", afesp_gpu_set_option(g_h, "frozen_core", s.frozen_core));
     // coeff(mo,ao) column-major as the Fortran host holds canon_coeff: element (mo,ao) at mo + n*ao
     std::vector<double> coeff_f((size_t)n * n);
     for (int mo = 0; mo < n; ++mo)

@@ -55,6 +55,15 @@ const char* afesp_gpu_last_error(afesp_handle h); /* h may be NULL: error of the
  *   "gemm_tma_edge"            1 (default): the TMA kernel multiplies only ceil(M/8) row fragments (ragged last m-tile shared
  *                              evenly by the warps) and two instead of four DMMA groups for a K tail of <= 8; 0: pad (A/B tests)
  *   "spinorb_symmetry_tol"     abort threshold of the spin-orbital symmetry self-check (default 1e-12, see ccsd_init_info)
+ * Model:
+ *   "frozen_core"              number k of frozen doubly occupied spatial orbitals (default 0): MP2, CCSD and the triples
+ *                              correlate orbitals k..nbasis-1 only -- the same calculation as on the active-orbital
+ *                              integrals (orbitals k.., eps[k:], nocc-k occupied), since the canonical RHF Fock operator is
+ *                              diagonal.  Read by afesp_gpu_mp2_energy and afesp_gpu_ccsd_init when they are called;
+ *                              ccsd_init keeps it with the CC state, so finalize, the CR intermediates and the triples of
+ *                              that state use it whatever the option says later.  A negative or non-integer value is
+ *                              refused here (status 1); k >= nocc is refused by mp2_energy / ccsd_init (status 1).  With a
+ *                              communicator attached every rank sets the same value.
  *   "dist_ccsd", "dist_min_flops"   see the multi-GPU section below */
 int afesp_gpu_set_option(afesp_handle h, const char* key, double value);
 /* State of the TMA-staged GEMM path: *scope = value of "gemm_use_tma" in force; *selftest = 1 when the start-up
@@ -87,7 +96,7 @@ int afesp_gpu_mp2_energy(afesp_handle h, int nocc, const double* eps, double* e_
 
 /* CCSD: replaces do_ccsd_spatial (src/ccsd.f90:279-402) / do_ccsd_spinorb (src/ccsd.f90:71-277) ----------------- */
 /* init_cc + init_diis_cc_t + the first update_cc_energy: returns the "MP1" line (energy, sum dT2^2).
- * nocc = number of doubly occupied spatial orbitals (sys%nel/2) in both formulations.  diis_n_errmat = sys%ccsd_diis_n_errmat,
+ * nocc = number of doubly occupied spatial orbitals (sys%nel/2) in both formulations, frozen core included.  diis_n_errmat = sys%ccsd_diis_n_errmat,
  * 0..64 (< 2 switches DIIS off as src/ccsd.f90:593-595 does; the history costs 2 x diis_n_errmat amplitude-sized arrays). */
 int afesp_gpu_ccsd_init(afesp_handle h, int nocc, int restricted, const double* eps, int diis_n_errmat,
                         double* e_mp1, double* rmst2);
@@ -106,9 +115,11 @@ int afesp_gpu_ccsd_init_info(afesp_handle h, double info[4]);
 int afesp_gpu_ccsd_iterate(afesp_handle h, double* e_cc, double* rmst2);
 /* update_diis_cc (src/ccsd.f90:617-676): extrapolate the amplitudes in place. */
 int afesp_gpu_ccsd_diis(afesp_handle h);
-/* After convergence (src/ccsd.f90:366-393 / 252-269): T1 diagnostic (spin-free: sqrt(sum t1^2)/sqrt(nel)), the CR
- * intermediates when want_cr != 0, optional copies of t1(o,v) and t2(o,o,v,v).  Amplitudes and the integral
- * slices (T) needs stay on the device (the int_store_cc hand-over of the reference). */
+/* After convergence (src/ccsd.f90:366-393 / 252-269): T1 diagnostic (spin-free: sqrt(sum t1^2)/sqrt(nel), nel = 2(nocc-k)
+ * correlated electrons with k = "frozen_core"), the CR intermediates when want_cr != 0, optional copies of t1(o,v) and
+ * t2(o,o,v,v) over the active orbitals: o = nocc-k, v = nbasis-nocc (spin-free) or o = 2(nocc-k), v = 2(nbasis-nocc)
+ * (spin-orbital).  Amplitudes and the integral slices (T) needs stay on the device (the int_store_cc hand-over of the
+ * reference). */
 int afesp_gpu_ccsd_finalize(afesp_handle h, int want_cr, double* t1_diagnostic, double* t1, double* t2);
 
 /* Triples: replaces do_ccsd_t_spatial (src/ccsd.f90:2018-2293) / do_ccsd_t_spinorb (src/ccsd.f90:1812-1922) ------ */

@@ -39,6 +39,7 @@ def main():
     ap.add_argument("--iters", type=int, default=6)
     ap.add_argument("--spinorb", action="store_true")
     ap.add_argument("--diis", action="store_true", help="extrapolate between the compared iterations")
+    ap.add_argument("--frozen-core", type=int, default=0, help="frozen doubly occupied orbitals (option frozen_core)")
     args = ap.parse_args()
     rank, world, local = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"]), int(os.environ["LOCAL_RANK"])
     torch.cuda.set_device(local)
@@ -52,6 +53,8 @@ def main():
     dist.broadcast(uid, 0)
     gpu.comm_init(rank, world, bytes(uid.cpu().tolist()))
     gpu.set_option("dist_min_flops", 0.0)   # shard every GEMM wide enough, also at this small shape
+    if args.frozen_core:
+        gpu.set_option("frozen_core", args.frozen_core)   # every rank sets it, like the other collective arguments
 
     def chain(sharded):
         gpu.set_option("dist_ccsd", 1.0 if sharded else 0.0)
@@ -92,6 +95,7 @@ def main():
     dist.all_reduce(flag, op=dist.ReduceOp.MIN)
     if rank == 0:
         _REAL.write(json.dumps({"world": world, "nbf": n, "nocc": o, "spinorb": args.spinorb, "diis": args.diis,
+                                "frozen_core": args.frozen_core,
                                 "max_abs_err": dict(zip(names, errs)), "tol": dict(zip(names, tols)),
                                 "ranks_bit_identical": identical, "e_ccsd": float(got[2][-1]),
                                 "abs_err_energy_per_iteration_rank0": per_iter,
